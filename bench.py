@@ -32,6 +32,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
+import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 COARSE = dict(n_heads=20, n_layers=20, n_codebooks=4, n_conditioning_codebooks=0, embedding_dim=1280)
@@ -348,6 +349,25 @@ def secondary_rooflines(cfg, B, fam_ms, fam_n, fl, peaks, codec_ms):
     return out
 
 
+DUMP_BUDGET = 64_000_000  # bytes, .npy headers included
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor as out_dir/<name>.npy (float32).  When the total exceeds DUMP_BUDGET every array is cut to
+    its share by a fixed, seeded choice of flat indices (sorted), so two runs with the same arguments store the same
+    elements."""
+    os.makedirs(out_dir, exist_ok=True)
+    total = sum(t.numel() * 4 for t in arrays.values())
+    budget = DUMP_BUDGET - 4096 * len(arrays)
+    for name, t in arrays.items():
+        a = t.numpy().astype(np.float32, copy=False)
+        if total > budget:
+            keep = a.size * budget // total
+            idx = np.sort(np.random.default_rng(0).choice(a.size, size=keep, replace=False))
+            a = a.reshape(-1)[idx]
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def main():
     quiet_stdout()
     ap = argparse.ArgumentParser()
@@ -358,7 +378,14 @@ def main():
     ap.add_argument("--config", type=int, default=2, choices=sorted(CONFIGS), help="BASELINE.json configs[k]")
     ap.add_argument("--batch", type=int, default=None, help="clips per GPU (default = the named config)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0) to DIR/<name>.npy, float32, "
+                         f"at most {DUMP_BUDGET // 10**6} MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs records the b200 path's outputs")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -503,6 +530,8 @@ def main():
     ms = e0.elapsed_time(e1)
     launches = lib.vnb_launch_count() - launches0
     clk = clocks.stop()
+    # copied now: later calls may reuse the buffers the last timed step returned
+    dumped = {("audio" if cfg["codec"] else "tokens"): out.float().cpu()} if args.dump_outputs and rank == 0 else None
 
     # ---- end to end: host (pinned) inputs, H2D + D2H inside the timed region, public API ----
     barrier()
@@ -599,6 +628,8 @@ def main():
             line["cpu_baseline"] = {"value": v, "unit": "tokens/s", "cores": threads, "kind": "port",
                                     "sample": cpu_sample_text(cfg, parts, threads)}
         emit(line)
+        if dumped is not None:
+            dump_outputs(args.dump_outputs, dumped)
     if world > 1:
         dist.destroy_process_group()
 

@@ -1,13 +1,13 @@
 """TEST INFRASTRUCTURE — not product code.
 
-Import the *unmodified* reference modules from /root/reference through two tiny
-shims, so that the reference's own code can be executed as the ground truth
-when golden vectors are generated (oracle/gen_golden.py) and when the CPU
-restatement (oracle/vampnet_oracle.py) is pinned (tests/test_oracle_vs_reference.py).
+Import the *unmodified* reference modules from a checkout of the reference
+(VAMPNET_REFERENCE_ROOT) through two tiny shims, so that the reference's own code
+can be executed as the ground truth when golden vectors are generated
+(oracle/gen_golden.py).  The tests only read those stored vectors.
 
 Nothing is copied: the reference files are imported from where they lie.
-/root/reference exists only in the authoring container, never on the GPU box,
-so everything here is optional at run time (``available()`` says whether it is).
+Nothing outside golden generation needs the checkout (``available()`` says
+whether it is present).
 
 Shims (SURVEY.md §8c):
   * ``audiotools``  -> ml.BaseModel = nn.Module subclass with a .device

@@ -1,27 +1,15 @@
 """CPU: the repository's ``vampnet`` package is a drop-in for the reference's import surface (SURVEY.md §8b).
 
-The reference's OWN import lines are executed (read from /root/reference/app.py:16-17 when the checkout is present,
-otherwise the same two lines verbatim), then the hello.py:1-36 call sequence up to the first device computation runs
-against a synthetic model cache written in the reference's on-disk layout, codec checkpoint in the lac /
+The reference's OWN import lines are executed (its app.py:16-17, verbatim), then the hello.py:1-36 call sequence up
+to the first device computation runs against a synthetic model cache written in the reference's on-disk layout, codec checkpoint in the lac /
 descript-audio-codec key layout included.  Everything that computes needs the GPU and is covered by
 tests/test_gpu_dropin.py; here a CPU-resident Interface must refuse to compute (there is no CPU fallback)."""
-import os
 import sys
 
 import pytest
 import torch
 
-APP_IMPORTS = ["from vampnet.interface import Interface, signal_concat", "from vampnet import mask as pmask"]
-
-
-def reference_import_lines():
-    path = "/root/reference/app.py"
-    if os.path.exists(path):
-        lines = open(path).read().splitlines()
-        got = [lines[15].strip(), lines[16].strip()]   # app.py:16-17
-        assert got == APP_IMPORTS, got                 # the literal fallback below is what the reference says
-        return got
-    return APP_IMPORTS
+APP_IMPORTS = ["from vampnet.interface import Interface, signal_concat", "from vampnet import mask as pmask"]  # app.py:16-17
 
 
 @pytest.fixture()
@@ -37,7 +25,7 @@ def cache(tmp_path, monkeypatch):
 
 def test_reference_import_lines_resolve_to_this_repository(cache):
     ns = {}
-    for line in reference_import_lines():
+    for line in APP_IMPORTS:
         exec(line, ns)
     import vampnet_b200.interface
     import vampnet_b200.mask

@@ -21,6 +21,7 @@ import pytest
 import torch
 
 from oracle import vampnet_oracle as vo
+from oracle.gen_golden import load
 
 pytestmark = pytest.mark.gpu
 
@@ -54,7 +55,7 @@ def build(cfgd, seed=0, lora=False, cb_seed=1):
 @pytest.mark.parametrize("tag,cfgd,lora", [("coarse", TINY_COARSE, False), ("c2f", TINY_C2F, False),
                                            ("coarse_lora", TINY_COARSE, True)])
 def test_forward_vs_oracle_and_golden(golden_dir, tag, cfgd, lora):
-    g = np.load(os.path.join(golden_dir, f"forward_tiny_{tag}.npz"))
+    g = load(os.path.join(golden_dir, f"forward_tiny_{tag}.npz"))
     cfg, sd, model, cb, codec = build(cfgd, seed=int(g["weight_seed"]), lora=lora, cb_seed=int(g["codebook_seed"]))
     lat = torch.from_numpy(g["latents"])
     got = model(lat.cuda()).cpu()  # (B, V, S)

@@ -20,6 +20,7 @@ import pytest
 import torch
 
 from oracle import vampnet_oracle as vo
+from oracle.gen_golden import load
 from tests.test_gpu_parity import TINY_C2F, TINY_COARSE, build
 
 pytestmark = pytest.mark.gpu
@@ -56,7 +57,7 @@ def assert_decisions_exact_where_margin_allows(got_bsv, ref32_bsv, tag):
 @pytest.mark.parametrize("tag,cfgd,lora", [("coarse", TINY_COARSE, False), ("c2f", TINY_C2F, False),
                                            ("coarse_lora", TINY_COARSE, True)])
 def test_forward_decisions_vs_reference_golden(golden_dir, tag, cfgd, lora):
-    g = np.load(os.path.join(golden_dir, f"forward_tiny_{tag}.npz"))
+    g = load(os.path.join(golden_dir, f"forward_tiny_{tag}.npz"))
     cfg, sd, model, cb, codec = build(cfgd, seed=int(g["weight_seed"]), lora=lora, cb_seed=int(g["codebook_seed"]))
     got = model(torch.from_numpy(g["latents"]).cuda()).cpu()          # (B, V, S)
     ref32 = torch.from_numpy(g["logits"])                             # the reference's own fp32 output

@@ -1,119 +1,144 @@
-"""CPU: Interface orchestration (SURVEY.md §8 rows A1-A3 + build_mask) pinned against the REFERENCE'S OWN code.
+"""CPU: Interface orchestration (SURVEY.md §8 rows A1-A3 + build_mask) pinned against outputs of the REFERENCE'S OWN code.
 
-The reference's vampnet/interface.py is imported from /root/reference through oracle/ref_shims.py (its codec and
-beat-tracker imports are name-only stubs; nothing is copied).  A reference `Interface` object and ours are given the
-same stand-in models — `generate` is a deterministic pure function of (start_tokens, mask) — so the outputs of
-`coarse_vamp`, `coarse_to_fine`, `vamp` and `build_mask` must be identical tensors: chunking, edge anchors, padding,
-codebook stacking, time stretch, feedback passes, mask composition and RNG consumption.  The oracle's restatement
-(oracle/vampnet_oracle.py) is checked in the same breath, which is what lets the GPU tests rely on it on the box
-where /root/reference does not exist.  Skipped when the reference is not mounted."""
-import warnings
+``python -m oracle.gen_golden vs_reference`` gave a reference `Interface` object (its vampnet/interface.py, codec and
+beat-tracker imports as name-only stubs) the stand-in models and the inputs defined here — `generate` is a
+deterministic pure function of (start_tokens, mask) — and stored its results in tests/golden/vs_reference_interface.npz.
+The outputs of `coarse_vamp`, `coarse_to_fine`, `vamp` and `build_mask`, and the generate calls behind them, must be
+identical: chunking, edge anchors, padding, codebook stacking, time stretch, feedback passes, mask composition and
+RNG consumption.  The oracle's restatement (oracle/vampnet_oracle.py) is checked in the same breath."""
+import json
+import os
 
+import numpy as np
 import pytest
 import torch
 
-from oracle import ref_shims
 from oracle import vampnet_oracle as vo
 from tests.test_interface_cpu import MASK_TOKEN, StubCodec, StubModel, fake_generate, rand_case
 
-pytestmark = pytest.mark.skipif(not ref_shims.available(), reason="reference not mounted")
-
-
-@pytest.fixture(scope="module")
-def ref_mod():
-    mod = ref_shims.load_reference_interface()
-    yield mod
-    ref_shims.uninstall()
-
-
-def make_pair(ref_mod, coarse_s=0.6, c2f_s=0.25):
-    from vampnet_b200.interface import Interface
-
-    def models():
-        coarse, c2f = StubModel(4, 0, salt=5), StubModel(14, 4, salt=9)
-        coarse.chunk_size_s, c2f.chunk_size_s = coarse_s, c2f_s
-        return coarse, c2f
-    ours = Interface.from_models(StubCodec(), *models(), device="cpu", coarse_chunk_size_s=coarse_s,
-                                 coarse2fine_chunk_size_s=c2f_s)
-    ref = ref_mod.Interface.__new__(ref_mod.Interface)   # the reference constructor loads checkpoints from disk
-    torch.nn.Module.__init__(ref)
-    ref.codec = StubCodec()
-    ref.coarse, ref.c2f = models()
-    ref.device = "cpu"
-    return ours, ref
-
-
-def quiet(fn, *a, **k):
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")  # the reference opens torch.autocast("cuda") (interface.py:428) on a CPU build
-        return fn(*a, **k)
-
-
-@pytest.mark.parametrize("T", [1, 34, 35, 36, 83, 140])
-def test_coarse_vamp(ref_mod, T):
-    ours, ref = make_pair(ref_mod)
-    z, mask = rand_case(2, T, seed=T)
-    if T > 70:
-        mask[:, :, 70:] = 1
-    want, want_start = quiet(ref.coarse_vamp, z, mask, return_mask=True, temperature=0.7)
-    got, got_start = ours.coarse_vamp(z, mask, return_mask=True, temperature=0.7)
-    assert torch.equal(got, want) and torch.equal(got_start, want_start)
-    o, o_start = vo.coarse_vamp(z, mask, 4, ours.s2t(0.6), MASK_TOKEN, lambda s, m: fake_generate(s, m, 5))
-    assert torch.equal(o, want) and torch.equal(o_start, want_start)
-    assert [c["kwargs"] for c in ours.coarse.calls] == [c["kwargs"] for c in ref.coarse.calls]
-    assert [c["shape"] for c in ours.coarse.calls] == [c["shape"] for c in ref.coarse.calls]
-
-
-@pytest.mark.parametrize("T,n_in", [(15, 14), (29, 14), (30, 4), (47, 14), (1, 4)])
-def test_coarse_to_fine(ref_mod, T, n_in):
-    ours, ref = make_pair(ref_mod)
-    z, mask = rand_case(2, T, seed=100 + T)
-    z = z[:, :n_in]
-    want, want_start = quiet(ref.coarse_to_fine, z, mask=mask, return_mask=True)
-    got, got_start = ours.coarse_to_fine(z, mask=mask, return_mask=True)
-    assert torch.equal(got, want) and torch.equal(got_start, want_start)
-    o, o_start = vo.coarse_to_fine(z, mask, 14, 4, ours.s2t(0.25), MASK_TOKEN, lambda s, m: fake_generate(s, m, 9))
-    assert torch.equal(o, want) and torch.equal(o_start, want_start)
-    assert torch.equal(ours.coarse_to_fine(z, mask=None), quiet(ref.coarse_to_fine, z, mask=None))
-    sig = lambda calls: [(c["time_steps"], c["shape"], c["kwargs"]) for c in calls]  # noqa: E731
-    assert sig(ours.c2f.calls) == sig(ref.c2f.calls)
-
-
-@pytest.mark.parametrize("batch,feedback,stretch,T", [(1, 1, 1, 83), (3, 1, 1, 40), (2, 2, 1, 61), (2, 3, 2, 37),
-                                                       (1, 1, 3, 20)])
-def test_vamp(ref_mod, batch, feedback, stretch, T):
-    ours, ref = make_pair(ref_mod)
-    z, mask = rand_case(1, T, seed=7 * T + batch)
-    kw = dict(batch_size=batch, feedback_steps=feedback, time_stretch_factor=stretch, return_mask=True, temperature=1.3)
-    want, want_mask = quiet(ref.vamp, z, mask, **kw)
-    got, got_mask = ours.vamp(z, mask, **kw)
-    assert torch.equal(got, want) and torch.equal(got_mask, want_mask)
-    o, o_mask = vo.vamp(z, mask, batch, feedback, stretch, 4, 14, 4, ours.s2t(0.6), ours.s2t(0.25), MASK_TOKEN,
-                        lambda s, m: fake_generate(s, m, 5), lambda s, m: fake_generate(s, m, 9))
-    assert torch.equal(o, want) and torch.equal(o_mask, want_mask)
-    assert [c["kwargs"] for c in ours.c2f.calls] == [c["kwargs"] for c in ref.c2f.calls]
-
-
-@pytest.mark.parametrize("kw", [
+COARSE_S, C2F_S = 0.6, 0.25
+COARSE_T = [1, 34, 35, 36, 83, 140]
+C2F_CASES = [(15, 14), (29, 14), (30, 4), (47, 14), (1, 4)]
+VAMP_CASES = [(1, 1, 1, 83), (3, 1, 1, 40), (2, 2, 1, 61), (2, 3, 2, 37), (1, 1, 3, 20)]
+BUILD_MASK_KW = [
     dict(),
     dict(rand_mask_intensity=0.7, periodic_prompt=5, periodic_prompt_width=2, upper_codebook_mask=4),
     dict(prefix_s=0.3, suffix_s=0.2, periodic_prompt=0, _dropout=0.3, ncc=1),
     dict(rand_mask_intensity=0.0, periodic_prompt=3, upper_codebook_mask=14),
-])
-def test_build_mask(ref_mod, kw):
-    ours, ref = make_pair(ref_mod)
+]
+UNIT_SECONDS = (0.0, 0.1, 1.0, 3.0, 10.0, 13.37)
+
+
+def stub_models():
+    coarse, c2f = StubModel(4, 0, salt=5), StubModel(14, 4, salt=9)
+    coarse.chunk_size_s, c2f.chunk_size_s = COARSE_S, C2F_S
+    return coarse, c2f
+
+
+def calls(model, keys):
+    """The generate calls a stand-in model saw, as plain JSON data."""
+    return json.dumps([{k: c[k] for k in keys} for c in model.calls])
+
+
+# Each case runs one entry point on an Interface (ours, or the reference's when the golden file is written) and
+# returns its results by name: token tensors, and the generate calls as JSON.
+def coarse_vamp_case(iface, T):
+    z, mask = rand_case(2, T, seed=T)
+    if T > 70:
+        mask[:, :, 70:] = 1
+    out, start = iface.coarse_vamp(z, mask, return_mask=True, temperature=0.7)
+    return dict(out=out, start=start, calls=calls(iface.coarse, ("kwargs", "shape")))
+
+
+def coarse_to_fine_case(iface, T, n_in):
+    z, mask = rand_case(2, T, seed=100 + T)
+    z = z[:, :n_in]
+    out, start = iface.coarse_to_fine(z, mask=mask, return_mask=True)
+    no_mask = iface.coarse_to_fine(z, mask=None)
+    return dict(out=out, start=start, no_mask=no_mask, calls=calls(iface.c2f, ("time_steps", "shape", "kwargs")))
+
+
+def vamp_case(iface, batch, feedback, stretch, T):
+    z, mask = rand_case(1, T, seed=7 * T + batch)
+    out, out_mask = iface.vamp(z, mask, batch_size=batch, feedback_steps=feedback, time_stretch_factor=stretch,
+                               return_mask=True, temperature=1.3)
+    return dict(out=out, mask=out_mask, calls=calls(iface.c2f, ("kwargs",)))
+
+
+def build_mask_case(iface, i):
     z, _ = rand_case(2, 97, seed=3)
     torch.manual_seed(11)
-    want = ref.build_mask(z, **kw)
-    state_ref = torch.get_rng_state()
-    torch.manual_seed(11)
-    got = ours.build_mask(z, **kw)
-    assert torch.equal(got, want)
-    assert torch.equal(torch.get_rng_state(), state_ref)  # the same draws were consumed in the same order
+    mask = iface.build_mask(z, **BUILD_MASK_KW[i])
+    return dict(mask=mask, rng=torch.get_rng_state())
 
 
-def test_units(ref_mod):
-    ours, ref = make_pair(ref_mod)
-    for s in (0.0, 0.1, 1.0, 3.0, 10.0, 13.37):
-        assert ours.s2t(s) == ref.s2t(s) and ours.s2t2s(s) == ref.s2t2s(s)
-    assert ours.t2s(575) == ref.t2s(575)
+def units(iface):
+    return json.dumps([[iface.s2t(s), iface.s2t2s(s)] for s in UNIT_SECONDS] + [iface.t2s(575)])
+
+
+def case_key(kind, *params):
+    return "_".join([kind] + [str(p) for p in params])
+
+
+@pytest.fixture(scope="module")
+def golden(golden_dir):
+    return np.load(os.path.join(golden_dir, "vs_reference_interface.npz"), allow_pickle=False)
+
+
+def ours():
+    from vampnet_b200.interface import Interface
+    return Interface.from_models(StubCodec(), *stub_models(), device="cpu", coarse_chunk_size_s=COARSE_S,
+                                 coarse2fine_chunk_size_s=C2F_S)
+
+
+def check(got, golden, key):
+    for name, v in got.items():
+        want = golden[f"{key}.{name}"]
+        if isinstance(v, str):
+            assert json.loads(v) == json.loads(str(want)), (key, name)
+        else:
+            assert torch.equal(v, torch.from_numpy(want).to(v.dtype)), (key, name)
+
+
+@pytest.mark.parametrize("T", COARSE_T)
+def test_coarse_vamp(golden, T):
+    iface = ours()
+    got = coarse_vamp_case(iface, T)
+    check(got, golden, case_key("coarse_vamp", T))
+    z, mask = rand_case(2, T, seed=T)
+    if T > 70:
+        mask[:, :, 70:] = 1
+    o, o_start = vo.coarse_vamp(z, mask, 4, iface.s2t(COARSE_S), MASK_TOKEN, lambda s, m: fake_generate(s, m, 5))
+    assert torch.equal(o, got["out"]) and torch.equal(o_start, got["start"])
+
+
+@pytest.mark.parametrize("T,n_in", C2F_CASES)
+def test_coarse_to_fine(golden, T, n_in):
+    iface = ours()
+    got = coarse_to_fine_case(iface, T, n_in)
+    check(got, golden, case_key("coarse_to_fine", T, n_in))
+    z, mask = rand_case(2, T, seed=100 + T)
+    o, o_start = vo.coarse_to_fine(z[:, :n_in], mask, 14, 4, iface.s2t(C2F_S), MASK_TOKEN,
+                                   lambda s, m: fake_generate(s, m, 9))
+    assert torch.equal(o, got["out"]) and torch.equal(o_start, got["start"])
+
+
+@pytest.mark.parametrize("batch,feedback,stretch,T", VAMP_CASES)
+def test_vamp(golden, batch, feedback, stretch, T):
+    iface = ours()
+    got = vamp_case(iface, batch, feedback, stretch, T)
+    check(got, golden, case_key("vamp", batch, feedback, stretch, T))
+    z, mask = rand_case(1, T, seed=7 * T + batch)
+    o, o_mask = vo.vamp(z, mask, batch, feedback, stretch, 4, 14, 4, iface.s2t(COARSE_S), iface.s2t(C2F_S), MASK_TOKEN,
+                        lambda s, m: fake_generate(s, m, 5), lambda s, m: fake_generate(s, m, 9))
+    assert torch.equal(o, got["out"]) and torch.equal(o_mask, got["mask"])
+
+
+@pytest.mark.parametrize("kw", BUILD_MASK_KW)
+def test_build_mask(golden, kw):
+    # the mask and the global RNG state afterwards: the same draws were consumed in the same order
+    check(build_mask_case(ours(), BUILD_MASK_KW.index(kw)), golden, case_key("build_mask", BUILD_MASK_KW.index(kw)))
+
+
+def test_units(golden):
+    assert json.loads(units(ours())) == json.loads(str(golden["units"]))

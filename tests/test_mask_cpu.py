@@ -1,10 +1,12 @@
-"""CPU: vampnet_b200.mask against the reference's vampnet/mask.py run live (authoring container) under the
-same torch seed, plus reference-free checks that run anywhere (including the reference's only fixture for this
-code, scratch/rms_mask.txt: period 7, 3 unmasked-able codebooks)."""
+"""CPU: vampnet_b200.mask against outputs of the reference's vampnet/mask.py under the same torch seed (stored in
+tests/golden/vs_reference_mask.npz), plus checks that need no reference output (including the reference's only fixture
+for this code, scratch/rms_mask.txt: period 7, 3 unmasked-able codebooks)."""
+import os
+
+import numpy as np
 import pytest
 import torch
 
-from oracle import ref_shims
 from vampnet_b200 import mask as pm
 
 
@@ -29,59 +31,59 @@ def test_apply_mask_and_inpaint():
         pm.apply_mask(x, m.int(), 1024)
 
 
-@pytest.mark.skipif(not ref_shims.available(), reason="/root/reference not present")
-def test_against_reference_mask_module():
-    _, rm, _ = ref_shims.load_reference()
-    try:
-        x = torch.randint(0, 1024, (3, 9, 57), generator=torch.Generator().manual_seed(0))
-        cases = [
-            lambda M: M.linear_random(x, 0.7),
-            lambda M: M.random(x, 0.3),
-            lambda M: M.inpaint(x, 4, 9),
-            lambda M: M.inpaint(x, 0, 0),
-            lambda M: M.periodic_mask(x, 7, 1, random_roll=True),
-            lambda M: M.periodic_mask(x, 5, 3, random_roll=True),
-            lambda M: M.periodic_mask(x, 0, 1),
-            lambda M: M.codebook_mask(M.codebook_unmask(M.full_mask(x), 2), 5),
-            lambda M: M.dropout(M.periodic_mask(x, 3, 1), 0.3),
-            lambda M: M.mask_or(M.inpaint(x, 2, 2), M.periodic_mask(x, 4, 1)),
-            lambda M: M.time_stretch_mask(x, 3),
-            lambda M: M.apply_mask(x, M.periodic_mask(x, 7, 1), 1024)[0],
-            lambda M: M._gamma(torch.linspace(0, 1, 13)),
-        ]
-        for i, fn in enumerate(cases):
-            torch.manual_seed(123 + i)
-            want = fn(rm)
-            torch.manual_seed(123 + i)
-            got = fn(pm)
-            assert torch.equal(want, got), f"case {i}"
-            # both leave the global RNG in the same state
-            assert torch.equal(torch.rand(3), (torch.manual_seed(123 + i), fn(rm), torch.rand(3))[2]) or True
-    finally:
-        ref_shims.uninstall()
+MASK_X_SEED, BUILD_X_SEED = 0, 1
+MASK_CASES = [
+    lambda M, x: M.linear_random(x, 0.7),
+    lambda M, x: M.random(x, 0.3),
+    lambda M, x: M.inpaint(x, 4, 9),
+    lambda M, x: M.inpaint(x, 0, 0),
+    lambda M, x: M.periodic_mask(x, 7, 1, random_roll=True),
+    lambda M, x: M.periodic_mask(x, 5, 3, random_roll=True),
+    lambda M, x: M.periodic_mask(x, 0, 1),
+    lambda M, x: M.codebook_mask(M.codebook_unmask(M.full_mask(x), 2), 5),
+    lambda M, x: M.dropout(M.periodic_mask(x, 3, 1), 0.3),
+    lambda M, x: M.mask_or(M.inpaint(x, 2, 2), M.periodic_mask(x, 4, 1)),
+    lambda M, x: M.time_stretch_mask(x, 3),
+    lambda M, x: M.apply_mask(x, M.periodic_mask(x, 7, 1), 1024)[0],
+    lambda M, x: M._gamma(torch.linspace(0, 1, 13)),
+]
 
 
-@pytest.mark.skipif(not ref_shims.available(), reason="/root/reference not present")
-def test_build_mask_rng_stream_matches_reference():
+def mask_case(M, i):
+    """Case i of MASK_CASES run with the mask module M (ours, or the reference's when the golden file is written)."""
+    x = torch.randint(0, 1024, (3, 9, 57), generator=torch.Generator().manual_seed(MASK_X_SEED))
+    torch.manual_seed(123 + i)
+    return MASK_CASES[i](M, x)
+
+
+def build_mask_stream(M):
+    """Interface.build_mask's composition of the pieces under torch.manual_seed(7), and the next draws after it."""
+    x = torch.randint(0, 1024, (2, 14, 100), generator=torch.Generator().manual_seed(BUILD_X_SEED))
+    torch.manual_seed(7)
+    m = M.linear_random(x, 1.0)
+    m = M.mask_and(m, M.inpaint(x, 0, 0))
+    m = M.mask_and(m, M.periodic_mask(x, 7, 1, random_roll=True))
+    m = M.dropout(m, 0.1)
+    m = M.codebook_unmask(m, 0)
+    return M.codebook_mask(m, 3, None), torch.rand(4)
+
+
+def _golden(golden_dir):
+    return np.load(os.path.join(golden_dir, "vs_reference_mask.npz"), allow_pickle=False)
+
+
+def test_against_reference_mask_module(golden_dir):
+    """Every piece of vampnet/mask.py against the reference's own outputs under the same torch seed
+    (tests/golden/vs_reference_mask.npz, written by ``python -m oracle.gen_golden vs_reference``)."""
+    g = _golden(golden_dir)
+    for i in range(len(MASK_CASES)):
+        got = mask_case(pm, i)
+        want = torch.from_numpy(g[f"case_{i}"])
+        assert got.dtype == want.dtype and torch.equal(got, want), f"case {i}"
+
+
+def test_build_mask_rng_stream_matches_reference(golden_dir):
     """Interface.build_mask composes the pieces; same seed -> same mask AND same RNG state afterwards."""
-    _, rm, _ = ref_shims.load_reference()
-    try:
-        x = torch.randint(0, 1024, (2, 14, 100), generator=torch.Generator().manual_seed(1))
-
-        def build(M):
-            m = M.linear_random(x, 1.0)
-            m = M.mask_and(m, M.inpaint(x, 0, 0))
-            m = M.mask_and(m, M.periodic_mask(x, 7, 1, random_roll=True))
-            m = M.dropout(m, 0.1)
-            m = M.codebook_unmask(m, 0)
-            return M.codebook_mask(m, 3, None)
-
-        torch.manual_seed(7)
-        a = build(rm)
-        ra = torch.rand(4)
-        torch.manual_seed(7)
-        b = build(pm)
-        rb = torch.rand(4)
-        assert torch.equal(a, b) and torch.equal(ra, rb)
-    finally:
-        ref_shims.uninstall()
+    g = _golden(golden_dir)
+    m, r = build_mask_stream(pm)
+    assert torch.equal(m, torch.from_numpy(g["build_mask"])) and torch.equal(r, torch.from_numpy(g["build_mask_next_rand"]))

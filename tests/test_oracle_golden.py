@@ -9,10 +9,11 @@ import pytest
 import torch
 
 from oracle import vampnet_oracle as vo
+from oracle.gen_golden import load
 
 
 def _load(golden_dir, name):
-    return np.load(os.path.join(golden_dir, name), allow_pickle=False)
+    return load(os.path.join(golden_dir, name))
 
 
 def _model(g, mode="fp32"):
